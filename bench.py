@@ -372,6 +372,26 @@ def reference_cuda_arm(args, config, rank, local_rank):
                               "(PyTorch gather/lerp around its rasterizer); compare with value_dropin of the default arm"}))
 
 
+# ----------------------------------------------------------------------------- outputs
+DUMP_MAX_ELEMENTS = 1 << 20       # per array: at most 8 MB each, so the seven arrays of a step stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy (integers and float64 as float64, everything else as float32), so that
+    two builds run with the same arguments can be compared output for output.  An array of more than DUMP_MAX_ELEMENTS
+    elements is written as the flat sample of that many elements at positions drawn with a fixed seed (sorted), the
+    same positions for every array of that size."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        dtype = torch.float32 if t.dtype in (torch.float32, torch.float16, torch.bfloat16) else torch.float64
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(dtype).cpu().numpy())
+
+
 # ----------------------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -390,6 +410,8 @@ def main():
                          "kernels over peer memory (the default on 2, 4 or 8 GPUs)")
     ap.add_argument("--classic", action="store_true",
                     help="also time the classic-formulation blend kernels (baseline/classic) on the same binned state")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -422,6 +444,8 @@ def main():
     import torch.distributed as dist
     if not torch.cuda.is_available():
         raise SystemExit("bench.py (impl ours) needs a CUDA device: there is no CPU fallback for this path")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes one process's outputs: run it on one GPU")
     torch.cuda.set_device(local_rank)
     dev = f"cuda:{local_rank}"
     if world > 1:
@@ -594,8 +618,23 @@ def main():
     torch.cuda.synchronize()
     l0 = _lib.launch_count()
     stats = []
-    ms_total = timed(step, args.steps, True, stats, graph_mode=gs is not None)         # <- `value`: profiler off
+    headline, last = step, []
+    if args.dump_outputs:
+        def headline(i, resident):
+            last[:] = [step(i, resident)]
+            return last[0]
+    ms_total = timed(headline, args.steps, True, stats, graph_mode=gs is not None)     # <- `value`: profiler off
     launches = _lib.launch_count() - l0
+    if args.dump_outputs:
+        loss, radii, _ = last[0]
+        if gs is not None:
+            rows = int(gs.status_dev[1].item())
+            outs = {"loss": loss, "image": gs.image, "radii": radii[:rows]}
+            outs.update({"grad_" + k: v for k, v in gs.grads.items()})
+        else:
+            outs = {"loss": loss, "radii": radii}
+            outs.update({"grad_" + k: getattr(scene, k).grad for k in ("means3D", "shs", "opacities", "scales", "rotations")})
+        dump_outputs(args.dump_outputs, outs)
     ms_e2e = timed(step, args.steps, False, graph_mode=gs is not None)
     clocks = sampler.stop() if rank == 0 else None
     if gs is not None:

@@ -1,11 +1,11 @@
 """TEST INFRASTRUCTURE ONLY.  Runs the reference's OWN, unmodified host code of the path --
-`gaussian_renderer.render()` / `render_post()` (/root/reference/gaussian_renderer/__init__.py:20-136, 138-292) --
+`gaussian_renderer.render()` / `render_post()` (gaussian_renderer/__init__.py:20-136, 138-292) --
 on top of the drop-in packages of this repo, with a stub `GaussianModel` / camera / pipe that carry exactly the
-attributes those two functions read.  Nothing is vendored: the reference checkout is put on sys.path where it
-exists (this container); on the GPU box it is absent and every user of this module skips.
+attributes those two functions read.  Nothing is vendored: the golden-data generators under tests/golden/ put a
+checkout of graphdeco-inria/hierarchical-3d-gaussians on sys.path, named by the H3DGS_REFERENCE environment variable;
+the tests themselves use only the stubs.
 
-Third-party packages the reference imports that are neither ours nor on this path (simple_knn, plyfile) are stubbed
-as in tests/test_reference_imports_cpu.py."""
+Third-party packages the reference imports that are neither ours nor on this path (simple_knn, plyfile) are stubbed."""
 import math
 import os
 import sys
@@ -13,11 +13,11 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ.get("H3DGS_REFERENCE", "")
 
 
 def have_reference():
-    return os.path.isfile(os.path.join(REF, "gaussian_renderer", "__init__.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "gaussian_renderer", "__init__.py"))
 
 
 def import_reference_renderer():
